@@ -1,7 +1,7 @@
 """Headline benchmark: forward images/sec of a tfimm classifier on N B200 GPUs (one node).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--model vit_base_patch16_224]
-                    [--batch 256] [--impl b200|reference]
+                    [--batch 256] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward pass of the model over one synthetic batch (``--batch`` images per GPU,
@@ -13,6 +13,12 @@ SM clocks sampled during the timed region.
 
 ``--impl reference`` times the CPU stand-in for the reference (the torch-CPU oracle restatement;
 TensorFlow is not installed in this image, see BASELINE.md section 3) on the same config.
+
+``--dump-outputs DIR`` writes, after the timed steps, the logits of the last timed step of every model as
+``DIR/<model>.npy`` (and of the end-to-end path as ``DIR/<model>_e2e.npy``), float32.  Inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output.  Compare with a bf16 tolerance: the
+depthwise kernels sum the squeeze-excite pooling with atomics, so EfficientNet logits can differ from run to run by a
+bf16 rounding step (measured on one B200, 1000 W power limit: 2 of 256 rows, up to 6e-4 of max|logit|).
 """
 import argparse
 import json
@@ -39,6 +45,10 @@ WORK = {
     "swin_base_patch4_window7_224": {"gflop": 30.86, "mb": 140.2, "bound": "hbm"},
     "efficientnet_b4": {"gflop": 8.79, "mb": 322.5, "bound": "hbm"},
 }
+
+
+# --dump-outputs writes at most this much; an output over its share keeps a fixed, seeded sample of its rows
+DUMP_BYTES = 64 << 20
 
 
 def _peaks():
@@ -169,7 +179,7 @@ def cpu_oracle_throughput(model_name, batch, iters, warmup=1):
     with torch.no_grad():
         for i in range(warmup + iters):
             t0 = time.perf_counter()
-            mod.forward(cfg, w, x)
+            y = mod.forward(cfg, w, x)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
@@ -177,7 +187,7 @@ def cpu_oracle_throughput(model_name, batch, iters, warmup=1):
     return {"value": batch / med, "unit": "images/sec", "cores": cores, "kind": "port",
             "sample": f"{model_name} fp32 forward, batch {batch}, median of {iters} after {warmup} warm-up "
                       f"(torch-CPU oracle restatement; TensorFlow is not installed)",
-            "ms_per_step": med * 1e3}
+            "ms_per_step": med * 1e3, "last_output": y}
 
 
 def run_reference(args):
@@ -195,7 +205,24 @@ def run_reference(args):
         "cpu_baseline": {k: res[k] for k in ("value", "unit", "cores", "kind", "sample")},
         "e2e": {"value": res["value"], "unit": "images/sec", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {args.model: res["last_output"]})
     print(json.dumps(line))
+
+
+def dump_outputs(directory, arrays):
+    """Writes {name: tensor} as ``<directory>/<name>.npy`` (float32), DUMP_BYTES in all at most."""
+    import numpy as np
+
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            keep = max(1, share // a[0].nbytes)
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(out / f"{name}.npy", np.ascontiguousarray(a))
 
 
 def _random_weights(model, torch, np):
@@ -281,11 +308,12 @@ def measure_model(model_name, args, ctx, sampler, with_roofline=True):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step(x_dev)
+        logits = step(x_dev)
     drain()
     e1.record()
     barrier()
     ms_local = e0.elapsed_time(e1)
+    outputs = {model_name: logits.float().cpu()} if (args.dump_outputs and rank == 0) else {}
     launches = ops.launch_count - launches0
     clocks = sampler.window(mark) if sampler is not None else None
     per_rank_ms = [ms_local / args.steps]
@@ -330,6 +358,8 @@ def measure_model(model_name, args, ctx, sampler, with_roofline=True):
     pipe.synchronize()
     barrier()
     e2e_ms = e0.elapsed_time(e1)
+    if outputs:
+        outputs[f"{model_name}_e2e"] = out_host.clone()
     if world > 1:
         t = torch.tensor([e2e_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -350,7 +380,7 @@ def measure_model(model_name, args, ctx, sampler, with_roofline=True):
                 "input": str(e2e_dtype).replace("torch.", ""),
                 "pipeline": "tfimm.serving.InferencePipeline depth 2 (H2D of step i+1 overlaps forward of step i)",
                 "d2h_bytes_per_step": out_host.numel() * 4, "ms_per_step": e2e_ms / args.steps},
-        "gpu_launches": launches, "roofline": roof,
+        "gpu_launches": launches, "roofline": roof, "outputs": outputs,
     }
     del pipe, forward, model, x_dev, host, host_e2e
     torch.cuda.empty_cache()
@@ -378,6 +408,7 @@ def run_b200(args):
     sampler.start()  # started before the warm-up: nvidia-smi needs ~1 s before its first sample
 
     head = measure_model(args.model, args, ctx, sampler)
+    outputs = dict(head["outputs"])
     # The other BASELINE.json configs, in the same run and the same JSON line ("extra"): the metric is quoted on
     # ViT-B/16 AND ConvNeXt-B; Swin-B and EfficientNet-B4 (native 380 px, 256 per GPU = 2048 over 8 GPUs) are
     # configs[3] and configs[4].  Every rank runs them (weak scaling + logits all-gather), rank 0 reports.
@@ -387,6 +418,7 @@ def run_b200(args):
             if name == args.model:
                 continue
             r = measure_model(name, args, ctx, sampler)
+            outputs.update(r["outputs"])
             extra[name] = {"value": r["value"], "unit": "images/sec", "ms_per_step": r["ms_per_step"],
                            "per_rank_ms_per_step": r["per_rank_ms_per_step"], "global_batch": world * args.batch,
                            "workload": r["workload"], "e2e": r["e2e"], "gpu_launches": r["gpu_launches"],
@@ -413,6 +445,8 @@ def run_b200(args):
             "clocks": head["clocks"], "e2e": head["e2e"], "gpu_launches": head["gpu_launches"],
             "roofline": head["roofline"], "cpu_baseline": cpu, "extra": extra,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -513,7 +547,11 @@ def main():
                     help="host image dtype of the end-to-end path (uint8 = raw pixels, preprocessing fused on device)")
     ap.add_argument("--no-graph", dest="graph", action="store_false",
                     help="launch kernels eagerly instead of replaying a captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the logits of the last timed step of every model to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -287,3 +287,39 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["value"] > 0
+
+
+def test_bench_dump_outputs_writes_the_timed_logits(tmp_path, monkeypatch):
+    """`--dump-outputs DIR` writes the last timed step's logits (seeded inputs: the same on every run) as float32 .npy,
+    and keeps a fixed sample of rows when the outputs exceed the size limit."""
+    import sys
+
+    root = Path(__file__).resolve().parent.parent
+    dumps = []
+    for run in ("a", "b"):
+        res = subprocess.run([sys.executable, str(root / "bench.py"), "--impl", "reference", "--steps", "2", "--warmup",
+                              "1", "--ref-batch", "2", "--model", "vit_tiny_patch16_224", "--dump-outputs",
+                              str(tmp_path / run)], capture_output=True, text=True, timeout=600, cwd=str(root))
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert sorted(p.name for p in (tmp_path / run).iterdir()) == ["vit_tiny_patch16_224.npy"]
+        dumps.append(np.load(tmp_path / run / "vit_tiny_patch16_224.npy"))
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (2, 1000)
+    assert np.array_equal(dumps[0], dumps[1])
+    from oracle import params
+    from oracle import vit as ovit
+
+    cfg = tfimm.models.model_config("vit_tiny_patch16_224")
+    want = ovit.forward(cfg, params.random_params(ovit.param_shapes(cfg), seed=0), params.test_images(2, 224, 224))
+    assert np.abs(dumps[0] - want.numpy()).max() <= 1e-4 * np.abs(want.numpy()).max()
+
+    sys.path.insert(0, str(root))
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096)
+    big = torch.arange(400 * 4, dtype=torch.float64).reshape(400, 4)
+    for run in ("c", "d"):
+        bench.dump_outputs(tmp_path / run, {"big": big, "small": torch.ones(3, 2)})
+    a = np.load(tmp_path / "c" / "big.npy")
+    assert a.dtype == np.float32 and a.shape == (128, 4) and np.array_equal(a, np.load(tmp_path / "d" / "big.npy"))
+    assert np.all(np.diff(a[:, 0]) > 0) and np.all(a[:, 0] % 4 == 0)  # whole rows of the original, in order
+    assert np.array_equal(np.load(tmp_path / "c" / "small.npy"), np.ones((3, 2), np.float32))
