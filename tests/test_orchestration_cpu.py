@@ -21,15 +21,11 @@ def _nerr(out, ref):
 
 
 @pytest.fixture
-def cpu_engine(monkeypatch):
-    from tfimm.models.model import Model
+def cpu_engine():
+    from oracle.launch_census import host_plan_on_cpu
 
-    def ensure_plan(self):
-        if self._plan is None:
-            self._plan = self._compile()
-        return self._plan
-
-    monkeypatch.setattr(Model, "_ensure_plan", ensure_plan)
+    with host_plan_on_cpu():
+        yield
 
 
 CASES = [
